@@ -19,6 +19,11 @@ the ranks by the operators themselves ("scaling": "strong").
 
 `--impl reference` times the CPU restatement of the reference algorithm (oracle/gp_oracle.py, the faithful chunked
 gp.eval(.., 'std') driver of SURVEY 8d) on the host cores, rank 0 only.
+
+`--dump-outputs DIR` writes, after the timed steps, what the last timed step of each leg handed its caller as
+DIR/<name>.npy (float64, rank 0): the arg-max (score, index or point) of every leg and, of the `value` leg's
+posterior, the log marginal likelihood, alpha and a fixed sample of L.  The inputs are seeded, so two builds run
+with the same arguments can be compared file by file.
 """
 import argparse
 import json
@@ -62,7 +67,12 @@ def parse_args():
   p.add_argument('--cpu-sample', type=int, default=24000)
   p.add_argument('--no-cpu-baseline', action='store_true')
   p.add_argument('--no-extras', action='store_true', help='skip the fp64-only / K_* / update side measurements')
-  return p.parse_args()
+  p.add_argument('--dump-outputs', metavar='DIR', default=None,
+                 help='write the outputs of the last timed step of every leg to DIR/<name>.npy')
+  args = p.parse_args()
+  if args.steps < 1:
+    p.error('--steps must be at least 1')
+  return args
 
 
 def dist_env():
@@ -398,10 +408,12 @@ class Workload(object):
     if self.cfg == 'headline':
       best, idx, _ = gp._fused_score(self.acq, self.cands_dev)      # returns after the device is done (16-byte read-back)
       self.local_ms.append(1e3 * (time.perf_counter() - t0))        # this rank's own work, before the collective
+      idx += self.rank * self.M
       if self.world > 1:
-        dfb_dist.all_reduce_argmax(best, idx + self.rank * self.M, self.dev)
+        best, idx = dfb_dist.all_reduce_argmax(best, idx, self.dev)
+      self.last_ret = (best, idx)
     else:
-      self.operator(gp, 'device')
+      self.last_ret = self.operator(gp, 'device')
     return gp
 
   def step_e2e(self):
@@ -410,9 +422,9 @@ class Workload(object):
     gp = self.make_gp()
     np.random.seed(7)
     if self.cfg == 'headline':
-      self.A.asy.ei(gp, self.anc('numpy'))
+      self.last_ret = self.A.asy.ei(gp, self.anc('numpy'))
     else:
-      self.operator(gp, 'numpy')
+      self.last_ret = self.operator(gp, 'numpy')
     return gp
 
   def step_e2e_device_rng(self):
@@ -421,10 +433,30 @@ class Workload(object):
     gp = self.make_gp()
     np.random.seed(7)
     if self.cfg == 'headline':
-      self.A.asy.ei(gp, self.anc('device'))
+      self.last_ret = self.A.asy.ei(gp, self.anc('device'))
     else:
-      self.operator(gp, 'device')
+      self.last_ret = self.operator(gp, 'device')
     return gp
+
+  def outputs(self, leg, gp, with_posterior):
+    """ What the step just run handed its caller, as float64 arrays named <leg>_<what>: the arg-max of the leg and,
+        with `with_posterior`, the posterior the step built (L as a fixed sample of 2^16 lower-triangle entries). """
+    ret = self.last_ret
+    if self.cfg == 'headline' and leg == 'device':
+      out = {'best_score': ret[0], 'best_index': ret[1]}
+    elif self.cfg == 'c5':
+      out = {'draw_max_values': ret[0], 'draw_argmax_indices': ret[1]}
+    else:
+      out = {'point': ret}
+    out = dict((leg + '_' + k, np.asarray(v, dtype=np.float64)) for k, v in out.items())
+    if with_posterior:
+      L = gp.L
+      rs = np.random.RandomState(0)
+      a, b = rs.randint(0, len(L), 1 << 16), rs.randint(0, len(L), 1 << 16)
+      out.update(posterior_lml=np.float64(gp.compute_log_marginal_likelihood()),
+                 posterior_alpha=np.asarray(gp.alpha, dtype=np.float64),
+                 posterior_L_sample=np.asarray(L[np.maximum(a, b), np.minimum(a, b)], dtype=np.float64))
+    return out
 
   def operator(self, gp, rng):
     A = self.A
@@ -450,6 +482,19 @@ class Workload(object):
     else:
       cand = self.global_m * self.d * 8
     return int(cand + train * self.world)
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def write_outputs(out_dir, arrays):
+  """ --dump-outputs: one float64 .npy per output, 64 MB at most in all. """
+  total = sum(a.nbytes for a in arrays.values())
+  if total > DUMP_LIMIT_BYTES:
+    raise ValueError('outputs to dump take %d bytes, more than %d' % (total, DUMP_LIMIT_BYTES))
+  os.makedirs(out_dir, exist_ok=True)
+  for name, a in sorted(arrays.items()):
+    np.save(os.path.join(out_dir, name + '.npy'), a)
 
 
 def run_ours(args):
@@ -478,11 +523,14 @@ def run_ours(args):
       dist.barrier()
     torch.cuda.synchronize(dev)
 
-  def timed(step, steps):
+  dump = {} if args.dump_outputs and rank == 0 else None
+
+  def timed(step, steps, leg=None):
     """ K steps; per step the larger of the device-event time and the host wall time of the same region (the
-        host view includes Python + ctypes + the candidate draw), so nothing is hidden. """
+        host view includes Python + ctypes + the candidate draw), so nothing is hidden.  With --dump-outputs, the
+        outputs of the last step of the named leg are kept, read back after its timed region. """
     times = []
-    for _ in range(steps):
+    for s in range(steps):
       flush.fill_(1.0)
       e0 = torch.cuda.Event(enable_timing=True); e1 = torch.cuda.Event(enable_timing=True)
       torch.cuda.synchronize(dev)
@@ -494,6 +542,8 @@ def run_ours(args):
       wall_ms = 1e3 * (time.perf_counter() - t0)
       times.append(max(e0.elapsed_time(e1), wall_ms))
       launches[0] += wl.post_of(gp).launch_count()
+      if dump is not None and leg is not None and s == steps - 1:
+        dump.update(wl.outputs(leg, gp, with_posterior=(leg == 'device')))
       del gp
     return times
 
@@ -503,23 +553,25 @@ def run_ours(args):
   sampler = ClockSampler(local)
   if rank == 0:
     sampler.start()
-  launches[0] = 0
-  wl.local_ms = []
-  t_dev = timed(wl.step_device, args.steps)
-  local_ms = float(np.mean(wl.local_ms)) if wl.local_ms else 0.0
-  n_launch = launches[0]
-  barrier()
-  wl.step_e2e()                                  # warm-up of the host path (pinned staging, thread start)
-  barrier()
-  t_e2e = timed(wl.step_e2e, args.steps)
-  barrier()
-  t_e2e_dev = []
-  if headline:
-    wl.step_e2e_device_rng()
+  try:
+    launches[0] = 0
+    wl.local_ms = []
+    t_dev = timed(wl.step_device, args.steps, 'device')
+    local_ms = float(np.mean(wl.local_ms)) if wl.local_ms else 0.0
+    n_launch = launches[0]
     barrier()
-    t_e2e_dev = timed(wl.step_e2e_device_rng, max(2, args.steps // 2))
+    wl.step_e2e()                                  # warm-up of the host path (pinned staging, thread start)
     barrier()
-  clocks = sampler.stop() if rank == 0 else None
+    t_e2e = timed(wl.step_e2e, args.steps, 'e2e')
+    barrier()
+    t_e2e_dev = []
+    if headline:
+      wl.step_e2e_device_rng()
+      barrier()
+      t_e2e_dev = timed(wl.step_e2e_device_rng, args.steps, 'e2e_device_candidates')
+      barrier()
+  finally:
+    clocks = sampler.stop() if rank == 0 else None
   ms_dev, ms_e2e = float(np.sum(t_dev)), float(np.sum(t_e2e))
   ms_e2e_dev = float(np.mean(t_e2e_dev)) if t_e2e_dev else 0.0
 
@@ -560,7 +612,7 @@ def run_ours(args):
     device.DEFAULT_OPTIONS['score_impl'] = 0
     wl.step_device()
     barrier()
-    ms_fp64 = float(np.sum(timed(wl.step_device, 2)))
+    ms_fp64 = float(np.sum(timed(wl.step_device, args.steps)))
     # the materialising K_* build of the fp64 path (the north-star's "K_* build vs HBM" figure), timed per
     # launch with the same event hooks
     gp = wl.make_gp()
@@ -615,6 +667,8 @@ def run_ours(args):
   value = wl.global_m * args.steps / (ms_dev * 1e-3)
   e2e_value = wl.global_m * args.steps / (ms_e2e * 1e-3)
 
+  if dump is not None:
+    write_outputs(args.dump_outputs, dump)
   if rank == 0:
     peaks = {}
     try:
@@ -708,8 +762,8 @@ def run_ours(args):
           'peak_source': 'live cuBLAS DGEMM 8192^3 burst on this GPU; DMMA issue peak measured live: %s TFLOP/s'
                          % issue.get('dmma_f64_tflops'), 'share_of_scoring': share}
       if not args.no_extras:
-        line['fp64_dmma_only'] = {'value': M * world * 2 / (ms_fp64 * 1e-3), 'unit': UNIT,
-                                  'note': 'same step with DFB200_SCORE=fp64 (no int8 path), 2 timed steps'}
+        line['fp64_dmma_only'] = {'value': M * world * args.steps / (ms_fp64 * 1e-3), 'unit': UNIT,
+                                  'note': 'same step with DFB200_SCORE=fp64 (no int8 path), %d timed steps' % args.steps}
         line['kstar_build_fp64'] = kstar_build_line(extras['kstar64'], N, peaks)
         line['posterior_update'] = extras.get('posterior_update')
     if not args.no_cpu_baseline and world == 1:

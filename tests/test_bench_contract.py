@@ -8,6 +8,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -68,3 +70,32 @@ def test_reference_arm_of_every_config():
     assert line['config']['n_train'] == 200 and 'workload' in line['config'] and 'model' not in line['config']
     assert line['cpu_baseline']['kind'] == 'port' and line['cpu_baseline']['value'] == line['value']
     assert line['e2e']['h2d_bytes_per_step'] == 0 and line['gpu_launches'] == 0
+
+
+@pytest.mark.gpu
+def test_dump_outputs_repeat_under_the_same_arguments(tmp_path):
+  """ `bench.py --dump-outputs DIR` on the GPU arm, twice with the same arguments: float64 .npy files of the last timed
+      step of every leg, the same values both times, and --steps timed steps in every leg. """
+  import numpy as np
+  dumps = []
+  for run in ('a', 'b'):
+    out_dir = str(tmp_path / run)
+    out = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py'), '--gpus', '1', '--steps', '3', '--warmup', '1',
+                          '--n-train', '1100', '--cands-per-gpu', '30000', '--no-extras', '--no-cpu-baseline',
+                          '--dump-outputs', out_dir],
+                         capture_output=True, text=True, env=dict(os.environ, PYTHONDONTWRITEBYTECODE='1'), timeout=900,
+                         cwd=ROOT)
+    assert out.returncode == 0, out.stderr[-3000:]
+    lines = [l for l in out.stdout.splitlines() if l.strip()]
+    assert len(lines) == 1, out.stdout
+    line = json.loads(lines[0])
+    assert line['steps'] == 3 and len(line['step_ms_each']['device']) == 3 and len(line['step_ms_each']['e2e']) == 3
+    dumps.append(dict((f[:-4], np.load(os.path.join(out_dir, f))) for f in sorted(os.listdir(out_dir))))
+  a, b = dumps
+  assert sorted(a) == sorted(b) == sorted(
+      ['device_best_score', 'device_best_index', 'e2e_point', 'e2e_device_candidates_point', 'posterior_lml',
+       'posterior_alpha', 'posterior_L_sample'])
+  assert a['posterior_alpha'].shape == (1100,) and a['e2e_point'].shape == (6,)
+  for name in a:
+    assert a[name].dtype == np.float64, name
+    np.testing.assert_allclose(a[name], b[name], rtol=1e-12, atol=0, err_msg=name)
